@@ -15,6 +15,7 @@ import ctypes
 import gc
 import json
 import os
+import shutil
 import subprocess
 import sys
 import tempfile
@@ -55,7 +56,12 @@ def parse():
     ap.add_argument("--phases", action="store_true", help="diagnostic: per-phase host wall times of every rank on stderr (adds syncs)")
     ap.add_argument("--root-upload", action="store_true",
                     help="N>1: rank 0 uploads all reads and broadcasts them (default: every rank uploads its slice, NCCL all-gather)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (N>1: DIR/rank<r>/); "
+                         "same arguments -> same inputs, so two builds can be compared output for output")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     if a.total_reads:
         assert a.total_reads % (a.gpus * a.gen_chunk) == 0, "--total-reads must be a multiple of --gen-chunk x GPUs"
         a.reads_per_gpu = a.total_reads // a.gpus
@@ -84,21 +90,52 @@ def workload_name(a, n_gpus):
         a.reads_per_gpu * n_gpus // 1_000_000, a.read_len, a.k, a.m)
 
 
-def bucket_xsum(stream, meta, wpt):
-    """Composable checksum of a shard's record stream: sum over its non-empty lv1 buckets of a keyed 64-bit digest of the
-    bucket's bytes (mod 2^64).  Buckets are disjoint between shards and batches, so the sums of N shards add up to the
-    1-GPU value; equal sums <=> equal per-bucket byte strings (up to digest collisions)."""
+def bucket_digests(stream, meta, wpt):
+    """uint64[65536]: a keyed 64-bit digest (blake2b, salt = bucket) of every non-empty lv1 bucket's bytes of the record
+    stream, 0 for an empty bucket."""
     import hashlib
     m = np.asarray(meta, dtype=np.int64)
     sizes = m[:, 0] * 2 + m[:, 2] * 2 + m[:, 1] * 4 * wpt
-    off, acc = 0, 0
+    out = np.zeros(len(m), dtype=np.uint64)
+    off = 0
     mv = memoryview(stream)
     for b in np.nonzero(sizes)[0]:
         n = int(sizes[b])
-        acc += int.from_bytes(hashlib.blake2b(mv[off:off + n], digest_size=8, salt=int(b).to_bytes(8, "little")).digest(), "little")
+        out[b] = int.from_bytes(hashlib.blake2b(mv[off:off + n], digest_size=8, salt=int(b).to_bytes(8, "little")).digest(), "little")
         off += n
     assert off == len(stream), "per-bucket table does not add up to the stream"
-    return acc & 0xFFFFFFFFFFFFFFFF
+    return out
+
+
+def bucket_xsum(stream, meta, wpt):
+    """Composable checksum of a shard's record stream: the sum of its bucket_digests (mod 2^64).  Buckets are disjoint
+    between shards and batches, so the sums of N shards add up to the 1-GPU value; equal sums <=> equal per-bucket byte
+    strings (up to digest collisions)."""
+    return int(bucket_digests(stream, meta, wpt).sum(dtype=np.uint64))
+
+
+DUMP_STREAM_SAMPLE = 8 << 20          # record-stream bytes in a --dump-outputs directory (32 MB as float32)
+
+
+def dump_outputs(d, last, stream, digests, seed, rank, world, buckets):
+    """--dump-outputs: what the last timed step returned -- stage 1's edge_counting, stage 2's per-bucket table and totals --
+    and its SdBG record stream (re-emitted from the same graph after the timed region: the timed path leaves the records in
+    HBM), as the per-bucket digests (hi, lo 32 bits) of the whole stream and its bytes (a seeded sample when it is larger
+    than DUMP_STREAM_SAMPLE / world).  A shard writes the rows of its own bucket range [b0, b1) of the tables, and rank 0
+    alone the whole-graph edge_counting, so that the files of all ranks stay at ~35 MB (32 MB sample, 3 MB tables) at any
+    N.  float64 holds every integer here exactly."""
+    b0, b1 = buckets
+    os.makedirs(d, exist_ok=True)
+    rec = np.frombuffer(stream, dtype=np.uint8)
+    n = DUMP_STREAM_SAMPLE // world
+    pick = np.sort(np.random.default_rng(seed).integers(0, len(rec), size=n)) if len(rec) > n else np.arange(len(rec))
+    arrays = {"bucket_table": last["meta"][b0:b1], "totals": last["totals"],
+              "stream_bucket_digest": np.stack([digests >> np.uint64(32), digests & np.uint64(0xFFFFFFFF)], axis=1)[b0:b1],
+              "stream_sample": rec[pick]}
+    if rank == 0 and last.get("edge_counting") is not None:              # min-count 1 has no stage 1
+        arrays["edge_counting"] = last["edge_counting"]
+    for name, x in arrays.items():
+        np.save(os.path.join(d, name + ".npy"), x.astype(np.float32 if x.dtype == np.uint8 else np.float64))
 
 
 # ------------------------------------------------------------------------------------------------ reference arm
@@ -154,11 +191,10 @@ def time_reference(prefix, a, work, tag, want_hash=False):
     return dt, int(res["meta"][:, 0].sum()), "port", 1, hashes
 
 
-def run_reference_arm(a):
+def run_reference_arm(a, work):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    work = tempfile.mkdtemp(prefix="mgta_bench_ref_")
     prefix, n = write_sample(a, work)
     times, edges, kind, cores, hashes = [], 0, "reference", 1, None
     for i in range(a.warmup + a.steps):
@@ -169,7 +205,7 @@ def run_reference_arm(a):
     ms = 1000.0 * sum(times) / len(times)
     value = edges / (ms / 1000.0)
     sample = "first %d reads of the %d-genome community (%d x %d bp), whole buildgraph, %d threads" % (n, sample_genomes(a), n, a.read_len, cores)
-    line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps,
+    line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": a.gpus, "steps": a.steps, "timed_steps": len(times),
             "warmup": a.warmup, "ms_per_step": ms, "higher_is_better": True, "scaling": "strong" if a.total_reads else "weak",
             "vs_baseline": None, "dtype": "u32", "data": "synthetic", "reads_per_s": n / (ms / 1000.0),
             "config": {"workload": workload_name(a, a.gpus), "reads": a.reads_per_gpu * a.gpus, "read_len": a.read_len, "k": a.k,
@@ -288,8 +324,14 @@ class DevBuf:
 
 def main():
     a = parse()
-    if a.impl == "reference":
-        return run_reference_arm(a)
+    work = tempfile.mkdtemp(prefix="mgta_bench_")          # the sample read library and the reference's files
+    try:
+        return run_reference_arm(a, work) if a.impl == "reference" else run_gpu_arm(a, work)
+    finally:
+        shutil.rmtree(work, ignore_errors=True)
+
+
+def run_gpu_arm(a, work):
 
     import torch
     import torch.distributed as dist
@@ -307,7 +349,6 @@ def main():
     L = a.read_len
 
     # ---- synthetic reads (rank 0 only; the other ranks receive them over NVLink)
-    work = tempfile.mkdtemp(prefix="mgta_bench_")
     sample_prefix, sample_n = os.path.join(work, "sample"), auto_sample(a)
     n_words = n_reads * L // 16 + 1
     # N = 1 (or --root-upload): rank 0 holds all reads, uploads them and broadcasts.  N > 1: every rank holds ITS slice of the
@@ -392,6 +433,7 @@ def main():
         return time.time()
 
     comm = shards.TorchComm(ctx, rank, world, dist, dev) if world > 1 else None
+    last = {}                                  # what the latest step returned (--dump-outputs)
 
     def step(e2e):
         """-> (edges of this shard, h2d bytes, d2h bytes).  N > 1: the library walks the sharded protocol
@@ -401,13 +443,11 @@ def main():
         t = mark("load", t)
         d2h = 0
         if a.m > 1:
-            if world > 1:
-                ctx.sharded(1, comm)
-            else:
-                ctx.stage1()
+            last["edge_counting"] = ctx.sharded(1, comm) if world > 1 else ctx.stage1()
             t = mark("stage1", t)
         collect = "count" if e2e else False
         nbytes, meta, totals = ctx.sharded(2, comm, collect=collect) if world > 1 else ctx.stage2(collect=collect)
+        last["meta"], last["totals"] = meta, totals
         if e2e:
             d2h = nbytes + meta[slice(*ctx.shard_range())].nbytes
         mark("stage2", t)
@@ -453,10 +493,17 @@ def main():
     # ---- parity evidence, outside every timed region: hashes of the records the last step's graph emits
     parity = {}
     wpt = (2 * a.k + 31) // 32
-    if not a.no_hash:
+    if not a.no_hash or a.dump_outputs:
         with torch.cuda.stream(stream):
             h_stream, h_meta, h_totals = ctx.sharded(2, comm, collect=True) if world > 1 else ctx.stage2(collect=True)
-        xs = bucket_xsum(h_stream, h_meta, wpt)
+        assert np.array_equal(h_meta, last["meta"]) and np.array_equal(h_totals, last["totals"]), \
+            "stage 2 emitted again differs from the last timed step"
+        digests = bucket_digests(h_stream, h_meta, wpt)
+        if a.dump_outputs:
+            dump_outputs(a.dump_outputs if world == 1 else os.path.join(a.dump_outputs, "rank%d" % rank), last, h_stream, digests,
+                         a.seed, rank, world, ctx.shard_range())
+    if not a.no_hash:
+        xs = int(digests.sum(dtype=np.uint64))
         part = torch.tensor([xs & 0xFFFFFFFF, xs >> 32, len(h_stream), int(h_meta[:, 0].sum()), int(h_meta[:, 1].sum())], dtype=torch.int64, device=dev)
         if world > 1:
             dist.all_reduce(part, op=dist.ReduceOp.SUM)
@@ -603,6 +650,7 @@ def main():
                 parity["full"] = {"reads": n_reads, "gpu": mine, "reference": full_h, "ok": mine == full_h, "reference_seconds": dtf,
                                   "reference_cores": coresf, "reference_edges_per_s": ef / dtf, "reference_reads_per_s": n_reads / dtf}
         line = {"metric": METRIC, "value": edges / (ms_dev / 1000.0), "unit": UNIT, "n_gpus": n_gpus, "steps": a.steps,
+                "timed_steps": {"device": len(outs), "e2e": len(outs_e2e)},
                 "warmup": a.warmup, "ms_per_step": ms_dev, "higher_is_better": True, "scaling": "strong" if a.total_reads else "weak",
                 "vs_baseline": None, "dtype": "u32", "data": "synthetic", "reads_per_s": n_reads / (ms_dev / 1000.0),
                 "config": {"workload": workload_name(a, n_gpus), "reads": n_reads, "read_len": L, "k": a.k, "min_count": a.m,

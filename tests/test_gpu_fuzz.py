@@ -1,10 +1,7 @@
-"""GPU, opt-in (MGTA_TEST_FUZZ=1): the CUDA path on the 52 seeded random read sets of tests/test_oracle_fuzz.py (ragged lengths,
-repeats, palindromes, k = 9 ... 127 around every word boundary, m = 1 ... 3, mercy) against the oracle, which that file
-pins on the reference binary run live.  Opt-in because it was written after this round's GPU budget was spent and has not
-been run on a GPU yet; its CPU counterpart (the product's __host__ __device__ logic on the same inputs) is
+"""GPU: the CUDA path on the 52 seeded random read sets of tests/test_oracle_fuzz.py (ragged lengths, repeats, palindromes,
+k = 9 ... 127 around every word boundary, m = 1 ... 3, mercy) against the oracle, which that file pins on the reference
+binary run live.  Its CPU counterpart (the product's __host__ __device__ logic on the same inputs) is
 tests/test_logic_cpu.py::test_product_logic_on_random_inputs."""
-import os
-
 import numpy as np
 import pytest
 
@@ -14,7 +11,6 @@ from oracle import oracle as O
 pytestmark = pytest.mark.gpu
 
 
-@pytest.mark.skipif(os.environ.get("MGTA_TEST_FUZZ") != "1", reason="opt-in: MGTA_TEST_FUZZ=1 (not yet run on a GPU)")
 def test_gpu_equals_the_oracle_on_random_inputs(tmp_path):
     import test_oracle_fuzz as F
     bad, ran = [], 0

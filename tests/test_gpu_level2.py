@@ -1,7 +1,7 @@
-"""GPU, opt-in (MGTA_TEST_LEVEL2=1): INTEGRATION.md "Level 2" end to end -- oracle/_ref/megagta_level2 (the reference's own
-option parser, loader and SdbgWriter around the C ABI, integration/level2_build_graph.cpp) builds the golden cases and its
-files are compared with the goldens of the unmodified reference.  Opt-in because it was written after this round's GPU
-budget was spent: its CPU half is tests/test_level2_integration_cpu.py, this half has not been run yet."""
+"""GPU: INTEGRATION.md "Level 2" end to end -- oracle/_ref/megagta_level2 (the reference's own option parser, loader and
+SdbgWriter around the C ABI, integration/level2_build_graph.cpp) builds the golden cases and its files are compared with the
+goldens of the unmodified reference.  The program is compiled from the reference's sources (oracle/Makefile), so the test
+skips where they are absent; its CPU half is tests/test_level2_integration_cpu.py."""
 import os
 import subprocess
 
@@ -15,7 +15,6 @@ ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 LEVEL2 = os.path.join(ROOT, "oracle", "_ref", "megagta_level2")
 
 
-@pytest.mark.skipif(os.environ.get("MGTA_TEST_LEVEL2") != "1", reason="opt-in: MGTA_TEST_LEVEL2=1 (not yet run on a GPU)")
 @pytest.mark.parametrize("variant", ["", "_raw"])      # SdbgWriter::write per record / append_raw per delivery (patched tree)
 @pytest.mark.parametrize("case", ["smoke_k31_m2", "adversarial_k27_m3"])
 def test_level2_writes_the_reference_files(case, variant, golden, read_lib, tmp_path):
