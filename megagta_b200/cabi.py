@@ -53,6 +53,11 @@ EXPORTS = ["mgta_ctx_create", "mgta_ctx_destroy", "mgta_last_error", "mgta_set_r
            "mgta_sdbg_create", "mgta_sdbg_destroy", "mgta_sdbg_last_error", "mgta_sdbg_append", "mgta_sdbg_sink", "mgta_sdbg_finish",
            "mgta_sdbg_header", "mgta_sdbg_array", "mgta_sdbg_copy", "mgta_stage2_into_sdbg", "mgta_pack_reads", "mgta_tools_last_error", "mgta_find_seeds"]
 
+# include/mgta_sdbg_query.h: kept apart from EXPORTS, which mirrors include/mgta_cuda.h
+QUERY_EXPORTS = ["mgta_sdbg_query_row_bytes", "mgta_sdbg_query"]
+(SQ_LOOKUP, SQ_LABEL, SQ_FORWARD, SQ_BACKWARD, SQ_OUTDEGREE, SQ_INDEGREE, SQ_OUTGOING, SQ_INCOMING, SQ_MULTIPLICITY,
+ SQ_REVCOMP) = range(1, 11)
+
 
 class SdbgHeader(ctypes.Structure):
     """mgta_sdbg_header_t"""
@@ -124,6 +129,8 @@ def load():
                                         ctypes.POINTER(ctypes.c_uint64)]
         lib.mgta_sdbg_sink.argtypes = [ctypes.c_void_p, ctypes.c_int32, ctypes.c_int32, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p]
         lib.mgta_words_per_key.argtypes = [ctypes.c_int, ctypes.c_int]
+        lib.mgta_sdbg_query_row_bytes.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(ctypes.c_uint64), ctypes.POINTER(ctypes.c_uint64)]
+        lib.mgta_sdbg_query.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_uint64]
         _lib = lib
     return _lib
 
@@ -334,6 +341,7 @@ class Sdbg:
         if rc != 0:
             raise MgtaError("mgta_sdbg_create failed (%d): no CUDA device? (there is no CPU fallback)" % rc)
         self.need_multiplicity = bool(need_multiplicity)
+        self.k, self.device = k, device
 
     def _check(self, rc, what):
         if rc != 0:
@@ -400,6 +408,91 @@ class Sdbg:
         out = np.zeros(n.value, dtype=np.uint8)
         self._check(self.lib.mgta_sdbg_copy(self.h, which, c, _p(out), n.value), "mgta_sdbg_copy")
         return out.view(dtype)
+
+    # ---- navigation queries (include/mgta_sdbg_query.h) ------------------------------------------------------------
+    def query(self, op, x):
+        """runs `op` (SQ_*) on every row of x: packed k-mers (uint32 [n, words]) for SQ_LOOKUP, edge ids (int64 [n]) for
+        the others.  x is a numpy array or a CUDA torch tensor, and the result is of the same kind (for a tensor it stays
+        on the device): int64 [n], int64 [n, 4] for SQ_OUTGOING / SQ_INCOMING, uint32 [n, words + 1] for SQ_LABEL
+        (int32 for a tensor; the last column is 1 for a tip node)."""
+        in_row, out_row = ctypes.c_uint64(), ctypes.c_uint64()
+        self._check(self.lib.mgta_sdbg_query_row_bytes(self.h, op, ctypes.byref(in_row), ctypes.byref(out_row)), "mgta_sdbg_query_row_bytes")
+        wpt = (2 * self.k + 31) // 32
+        cols = {SQ_LABEL: wpt + 1, SQ_OUTGOING: 4, SQ_INCOMING: 4}.get(op, 1)
+        if isinstance(x, np.ndarray):
+            x = np.ascontiguousarray(x, dtype=np.uint32 if op == SQ_LOOKUP else np.int64)
+            n = x.nbytes // in_row.value
+            if n * in_row.value != x.nbytes:
+                raise ValueError("input of %d bytes is not a whole number of %d-byte rows" % (x.nbytes, in_row.value))
+            out = np.empty((n, cols), dtype=np.uint32 if op == SQ_LABEL else np.int64)
+            self._check(self.lib.mgta_sdbg_query(self.h, op, _p(x) if n else None, n, _p(out) if n else None, out.nbytes), "mgta_sdbg_query")
+        else:
+            import torch
+            if not x.is_cuda or x.device.index != self.device:
+                raise ValueError("a tensor input must live on cuda:%d, the graph's device" % self.device)
+            x = x.contiguous()
+            if x.element_size() * x.numel() % in_row.value:
+                raise ValueError("input of %d bytes is not a whole number of %d-byte rows" % (x.element_size() * x.numel(), in_row.value))
+            n = x.element_size() * x.numel() // in_row.value
+            out = torch.empty((n, cols), dtype=torch.int32 if op == SQ_LABEL else torch.int64, device=x.device)
+            torch.cuda.current_stream(x.device).synchronize()      # x is written on torch's stream, the query runs on the graph's
+            self._check(self.lib.mgta_sdbg_query(self.h, op, x.data_ptr() if n else None, n, out.data_ptr() if n else None,
+                                                 out.numel() * 8 if op != SQ_LABEL else out.numel() * 4), "mgta_sdbg_query")
+        return out if cols > 1 else out.reshape(-1)
+
+    def lookup(self, kmers):
+        """packed k-mers -> the last edge of each node, or -1"""
+        return self.query(SQ_LOOKUP, kmers)
+
+    def label(self, edges):
+        return self.query(SQ_LABEL, edges)
+
+    def forward(self, edges):
+        return self.query(SQ_FORWARD, edges)
+
+    def backward(self, edges):
+        return self.query(SQ_BACKWARD, edges)
+
+    def outdegree(self, edges):
+        return self.query(SQ_OUTDEGREE, edges)
+
+    def indegree(self, edges):
+        return self.query(SQ_INDEGREE, edges)
+
+    def outgoing(self, edges):
+        return self.query(SQ_OUTGOING, edges)
+
+    def incoming(self, edges):
+        return self.query(SQ_INCOMING, edges)
+
+    def multiplicity(self, edges):
+        return self.query(SQ_MULTIPLICITY, edges)
+
+    def revcomp(self, edges):
+        return self.query(SQ_REVCOMP, edges)
+
+
+def pack_kmers(kmers, k):
+    """ACGT strings of length k -> uint32 [n, ceil(2k / 32)]: the first character in bits 31..30 of word 0, unused low bits 0"""
+    wpt = (2 * k + 31) // 32
+    if any(len(s) != k for s in kmers):
+        raise ValueError("every k-mer must have %d characters" % k)
+    codes = np.frombuffer("".join(kmers).encode(), dtype=np.uint8).reshape(len(kmers), k)
+    lut = np.full(256, 255, np.uint8)
+    lut[np.frombuffer(b"ACGT", np.uint8)] = np.arange(4, dtype=np.uint8)
+    c = lut[codes].astype(np.uint32)
+    if (c == 255).any():
+        raise ValueError("k-mers are over ACGT")
+    c = np.concatenate([c, np.zeros((len(kmers), wpt * 16 - k), np.uint32)], axis=1).reshape(len(kmers), wpt, 16)
+    return (c << (2 * np.arange(15, -1, -1, dtype=np.uint32))).sum(axis=2, dtype=np.uint32)
+
+
+def unpack_kmers(words, k):
+    """uint32 [n, >= ceil(2k / 32)] (LABEL rows may carry their tip column) -> ACGT strings of length k"""
+    w = np.asarray(words, dtype=np.uint32)[:, :(2 * k + 31) // 32]
+    c = (w[:, :, None] >> (2 * np.arange(15, -1, -1, dtype=np.uint32))) & 3
+    s = np.frombuffer(b"ACGT", np.uint8)[c.reshape(len(w), -1)[:, :k]]
+    return [r.tobytes().decode() for r in s]
 
 
 def pack_reads(seqs, device=0):
