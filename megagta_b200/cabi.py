@@ -57,6 +57,9 @@ EXPORTS = ["mgta_ctx_create", "mgta_ctx_destroy", "mgta_last_error", "mgta_set_r
 QUERY_EXPORTS = ["mgta_sdbg_query_row_bytes", "mgta_sdbg_query"]
 (SQ_LOOKUP, SQ_LABEL, SQ_FORWARD, SQ_BACKWARD, SQ_OUTDEGREE, SQ_INDEGREE, SQ_OUTGOING, SQ_INCOMING, SQ_MULTIPLICITY,
  SQ_REVCOMP) = range(1, 11)
+# include/mgta_sdbg_unitig.h
+UNITIG_EXPORTS = ["mgta_sdbg_unitigs", "mgta_sdbg_unitig_copy"]
+UNITIG_CYCLE, UNITIG_SELF_RC = 1, 2
 
 
 class SdbgHeader(ctypes.Structure):
@@ -131,6 +134,8 @@ def load():
         lib.mgta_words_per_key.argtypes = [ctypes.c_int, ctypes.c_int]
         lib.mgta_sdbg_query_row_bytes.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.POINTER(ctypes.c_uint64), ctypes.POINTER(ctypes.c_uint64)]
         lib.mgta_sdbg_query.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_uint64]
+        lib.mgta_sdbg_unitigs.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_uint64)]
+        lib.mgta_sdbg_unitig_copy.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_uint64]
         _lib = lib
     return _lib
 
@@ -471,6 +476,26 @@ class Sdbg:
     def revcomp(self, edges):
         return self.query(SQ_REVCOMP, edges)
 
+    # ---- unitigs (include/mgta_sdbg_unitig.h) ------------------------------------------------------------------------
+    def unitigs(self, device=False):
+        """the maximal non-branching paths of the graph, one of every reverse-complement pair -> (rows int64 [U, 6]:
+        first_edge, last_edge, n_edges, seq_offset, mult_sum, flags (UNITIG_CYCLE | UNITIG_SELF_RC); seq uint8 [chars]:
+        the ASCII sequences in row order).  numpy arrays, or CUDA tensors on the graph's device when device=True."""
+        n_rows, n_chars = ctypes.c_int64(), ctypes.c_uint64()
+        self._check(self.lib.mgta_sdbg_unitigs(self.h, ctypes.byref(n_rows), ctypes.byref(n_chars)), "mgta_sdbg_unitigs")
+        U, C = n_rows.value, n_chars.value
+        if device:
+            import torch
+            rows = torch.empty((U, 6), dtype=torch.int64, device="cuda:%d" % self.device)
+            seq = torch.empty(C, dtype=torch.uint8, device=rows.device)
+            torch.cuda.current_stream(rows.device).synchronize()     # the copy runs on the graph's stream
+            rp, sp = rows.data_ptr(), seq.data_ptr()
+        else:
+            rows, seq = np.empty((U, 6), np.int64), np.empty(C, np.uint8)
+            rp, sp = rows.ctypes.data, seq.ctypes.data
+        self._check(self.lib.mgta_sdbg_unitig_copy(self.h, rp if U else None, U * 48, sp if C else None, C), "mgta_sdbg_unitig_copy")
+        return rows, seq
+
 
 def pack_kmers(kmers, k):
     """ACGT strings of length k -> uint32 [n, ceil(2k / 32)]: the first character in bits 31..30 of word 0, unused low bits 0"""
@@ -493,6 +518,30 @@ def unpack_kmers(words, k):
     c = (w[:, :, None] >> (2 * np.arange(15, -1, -1, dtype=np.uint32))) & 3
     s = np.frombuffer(b"ACGT", np.uint8)[c.reshape(len(w), -1)[:, :k]]
     return [r.tobytes().decode() for r in s]
+
+
+def _host(a):
+    return a.cpu().numpy() if hasattr(a, "cpu") else np.asarray(a)
+
+
+def unitig_strings(rows, seq):
+    """rows and sequence of Sdbg.unitigs (numpy or torch) -> the ACGT string of every row"""
+    rows, seq = _host(rows), _host(seq)
+    ends = np.append(rows[1:, 3], len(seq)) if len(rows) else np.zeros(0, np.int64)
+    b = seq.tobytes()
+    return [b[o:e].decode() for o, e in zip(rows[:, 3].tolist(), ends.tolist())]
+
+
+def write_unitigs_fasta(path, rows, seq, min_len=0):
+    """the unitigs as plain FASTA (usable as the next k's `buildgraph --assist_seq`), those of at least min_len
+    characters: >unitig_<row> len=<chars> edges=<n> multi=<mult_sum / n, or na> flags=<flags>"""
+    rows = _host(rows)
+    with open(path, "w") as f:
+        for i, s in enumerate(unitig_strings(rows, seq)):
+            if len(s) < min_len:
+                continue
+            n, mult, flags = int(rows[i, 2]), int(rows[i, 4]), int(rows[i, 5])
+            f.write(">unitig_%d len=%d edges=%d multi=%s flags=%d\n%s\n" % (i, len(s), n, "%.2f" % (mult / n) if mult >= 0 else "na", flags, s))
 
 
 def pack_reads(seqs, device=0):

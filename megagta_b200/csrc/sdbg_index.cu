@@ -274,7 +274,8 @@ extern "C" void mgta_sdbg_destroy(mgta_sdbg *g) {
     cudaStreamSynchronize(g->stream);
     DevBuf *all[] = {&g->w, &g->last, &g->tip, &g->invalid, &g->multi1, &g->edge_multi, &g->tip_seq, &g->large_edge, &g->large_val,
                      &g->staging, &g->base, &g->meta, &g->w_minor, &g->w_major, &g->last_minor, &g->last_major, &g->tip_minor,
-                     &g->tip_major, &g->last_sel, &g->small, &g->q_bucket, &g->q_in, &g->q_out, &g->q_err};
+                     &g->tip_major, &g->last_sel, &g->small, &g->q_bucket, &g->q_in, &g->q_out, &g->q_err,
+                     &g->ut_rows, &g->ut_seq, &g->ut_edge, &g->ut_seg, &g->ut_jump};
     for (DevBuf *b : all) cudaFree(b->p);
     for (auto &b : g->w_sel) cudaFree(b.p);
     cudaFree(g->d_err);

@@ -1,5 +1,6 @@
-// sdbg_index.cuh -- the device SdBG shared by the index builder (sdbg_index.cu) and the navigation queries (sdbg_query.cu):
-// the state behind mgta_sdbg, and the rank arithmetic over its tables (layouts: sdbg_index.cu header comment).
+// sdbg_index.cuh -- the device SdBG shared by the index builder (sdbg_index.cu), the navigation queries (sdbg_query.cu) and
+// the unitigs (sdbg_unitig.cu): the state behind mgta_sdbg, and the rank arithmetic over its tables (layouts: sdbg_index.cu
+// header comment).
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
@@ -62,6 +63,11 @@ struct mgta_sdbg {
     // first edge of every lv1 bucket (65536 + 1 entries, from the deliveries' bucket tables), and the queries' buffers
     std::vector<long long> bucket_start = std::vector<long long>(65537, 0);
     mgta_sdbg_impl::DevBuf q_bucket, q_in, q_out, q_err;
+    // unitigs (sdbg_unitig.cu): the rows and sequence of the last mgta_sdbg_unitigs, and its scratch (freed when it returns)
+    mgta_sdbg_impl::DevBuf ut_rows, ut_seq, ut_edge, ut_seg, ut_jump;
+    bool ut_ready = false;
+    long long ut_n_rows = 0;
+    unsigned long long ut_n_chars = 0;
 };
 
 #define SCK(call)                                                                                        \
