@@ -194,3 +194,17 @@ def tandem_reads(seed=3, read_len=120, units=("A", "AC", "AACGT", "ACCGATT", "AG
         reads += [rep, (3 - rep)[::-1]]
     reads += [rng.integers(0, 4, size=read_len, dtype=np.uint8) for _ in range(6)]
     return read_dict(reads)
+
+
+PALINDROMIC_UNITS = ("A", "AT", "ACGT", "AC", "AACGT", "CG")    # AT, ACGT, CG: cycles that are their own reverse complement
+
+
+def shape_reads(shape, k):
+    """the read set of a hard shape ("long", "circular", "tandem") with reads long enough for k: at least k + 60 bases;
+    250 for the circular genome at k > 100, where 150 bp reads leave the cycle in pieces; tandem repeats of
+    PALINDROMIC_UNITS"""
+    if shape == "long":
+        return long_genome_reads(read_len=max(150, k + 60))
+    if shape == "circular":
+        return circular_genome_reads(read_len=250 if k > 100 else 150)
+    return tandem_reads(read_len=max(120, k + 60), units=PALINDROMIC_UNITS)

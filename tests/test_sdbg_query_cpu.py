@@ -39,6 +39,26 @@ def random_reads(seed, n_reads=300, read_len=90, genome=3000, polya=0, repeats=0
     return dict(seq=seq, start=start, n_reads=len(reads), max_len=int(lens.max()))
 
 
+RANDOM_KM = [(13, 1), (15, 2), (16, 3), (17, 2), (31, 1), (32, 2), (33, 3), (63, 2), (64, 1), (127, 2)]
+
+
+def matrix_reads(k, m):
+    """the random read set of the (k, m) cell of RANDOM_KM"""
+    return random_reads(1000 + k * 10 + m, read_len=max(90, k + 40), polya=4, repeats=3, palindromes=6)
+
+
+def fuzz_case(seed, d):
+    """the read set of test_oracle_fuzz.make_case(seed) (files under d), its assist reads appended when the case has any
+    -> (reads, k, m, need_mercy, n_short, the oracle's build_graph of it or None when it has no solid edge)"""
+    import test_oracle_fuzz as F
+    prefix, k, m, mercy, fa = F.make_case(seed, d)
+    rd, n_short = O.load_read_lib(prefix), None
+    if fa:
+        rd, n_short = O.with_assist(rd, fa)
+    res = O.build_graph(rd, k, m, need_mercy=mercy, n_short=n_short)
+    return rd, k, m, mercy, n_short, (res if int(res["meta"][:, 0].sum()) else None)
+
+
 def check_against_brute_force(rd, k, m, need_mercy=False, n_short=None, absent=2000, seed=0):
     res = O.build_graph(rd, k, m, need_mercy=need_mercy, n_short=n_short)
     ref = R.Restated(SO.build(res["stream"], np.asarray(res["meta"]), k, True), k)
@@ -104,10 +124,22 @@ def test_restatement_equals_brute_force_on_datasets(read_lib, ds, k, m):
     check_against_brute_force(rd, k, m)
 
 
-@pytest.mark.parametrize("k,m", [(13, 1), (15, 2), (16, 3), (17, 2), (31, 1), (32, 2), (33, 3), (63, 2), (64, 1), (127, 2)])
+@pytest.mark.parametrize("k,m", RANDOM_KM)
 def test_restatement_equals_brute_force_on_random_reads(k, m):
-    rd = random_reads(1000 + k * 10 + m, read_len=max(90, k + 40), polya=4, repeats=3, palindromes=6)
-    check_against_brute_force(rd, k, m, seed=k)
+    check_against_brute_force(matrix_reads(k, m), k, m, seed=k)
+
+
+@pytest.mark.parametrize("seed", range(52))
+def test_restatement_equals_brute_force_on_fuzz_inputs(seed, tmp_path):
+    """k = 9 ... 127 around every word boundary, ragged reads, errors, mercy and assist reads"""
+    rd, k, m, mercy, n_short, res = fuzz_case(seed, str(tmp_path))
+    if res is None:
+        pytest.skip("no solid edge")
+    check_against_brute_force(rd, k, m, need_mercy=mercy, n_short=n_short, absent=300, seed=seed)
+
+
+def test_most_fuzz_inputs_have_a_graph(tmp_path):
+    assert sum(fuzz_case(seed, str(tmp_path))[-1] is not None for seed in range(52)) >= 40
 
 
 def test_mercy_and_assist_reads(read_lib, data_dir):

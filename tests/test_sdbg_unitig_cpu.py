@@ -16,7 +16,7 @@ import sdbg_query_ref as R
 import sdbg_unitig_ref as U
 from oracle import oracle as O
 from oracle import sdbg_oracle as SO
-from test_sdbg_query_cpu import random_reads
+from test_sdbg_query_cpu import RANDOM_KM, fuzz_case, matrix_reads, random_reads
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -47,10 +47,17 @@ def test_restated_unitigs_equal_brute_force_on_datasets(read_lib, ds, k, m):
     check_against_brute_force(rd, k, m)
 
 
-@pytest.mark.parametrize("k,m", [(13, 1), (15, 2), (16, 3), (17, 2), (31, 1), (32, 2), (33, 3), (63, 2), (64, 1), (127, 2)])
+@pytest.mark.parametrize("k,m", RANDOM_KM)
 def test_restated_unitigs_equal_brute_force_on_random_reads(k, m):
-    rd = random_reads(1000 + k * 10 + m, read_len=max(90, k + 40), polya=4, repeats=3, palindromes=6)
-    check_against_brute_force(rd, k, m)
+    check_against_brute_force(matrix_reads(k, m), k, m)
+
+
+@pytest.mark.parametrize("seed", range(52))
+def test_restated_unitigs_equal_brute_force_on_fuzz_inputs(seed, tmp_path):
+    rd, k, m, mercy, n_short, res = fuzz_case(seed, str(tmp_path))
+    if res is None:
+        pytest.skip("no solid edge")
+    check_against_brute_force(rd, k, m, need_mercy=mercy, n_short=n_short)
 
 
 def test_mercy_and_assist_reads(read_lib, data_dir):
@@ -82,6 +89,19 @@ def test_tandem_repeats_give_short_cycles():
     _, rows, _ = check_against_brute_force(U.tandem_reads(), 21, 1)
     cyc = rows[rows[:, 5] & U.CYCLE == U.CYCLE]
     assert sorted(cyc[:, 2].tolist()) == [1, 2, 5, 7, 13]            # poly-A is a self-loop (and poly-T its partner)
+
+
+@pytest.mark.parametrize("k", [16, 64, 127])
+def test_circular_genome_at_large_and_even_k(k):
+    _, rows, _ = check_against_brute_force(U.shape_reads("circular", k), k, 1)
+    cyc = rows[rows[:, 5] & U.CYCLE == U.CYCLE]
+    assert len(cyc) == 1 and cyc[0, 2] == 5000
+
+
+@pytest.mark.parametrize("k", [16, 64, 127])
+def test_palindromic_tandem_repeats_give_self_reverse_complement_cycles(k):
+    _, rows, _ = check_against_brute_force(U.shape_reads("tandem", k), k, 1)
+    assert ((rows[:, 5] == U.CYCLE | U.SELF_RC).sum()) == 3            # the cycles of AT, ACGT and CG
 
 
 # ---- the C ABI of include/mgta_sdbg_unitig.h -----------------------------------------------------------------------
