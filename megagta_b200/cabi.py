@@ -60,6 +60,8 @@ QUERY_EXPORTS = ["mgta_sdbg_query_row_bytes", "mgta_sdbg_query"]
 # include/mgta_sdbg_unitig.h
 UNITIG_EXPORTS = ["mgta_sdbg_unitigs", "mgta_sdbg_unitig_copy"]
 UNITIG_CYCLE, UNITIG_SELF_RC = 1, 2
+# include/mgta_sdbg_unitig_graph.h
+UNITIG_GRAPH_EXPORTS = ["mgta_sdbg_unitig_links", "mgta_sdbg_unitig_link_copy"]
 
 
 class SdbgHeader(ctypes.Structure):
@@ -136,6 +138,8 @@ def load():
         lib.mgta_sdbg_query.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_uint64]
         lib.mgta_sdbg_unitigs.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64), ctypes.POINTER(ctypes.c_uint64)]
         lib.mgta_sdbg_unitig_copy.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64, ctypes.c_void_p, ctypes.c_uint64]
+        lib.mgta_sdbg_unitig_links.argtypes = [ctypes.c_void_p, ctypes.POINTER(ctypes.c_int64)]
+        lib.mgta_sdbg_unitig_link_copy.argtypes = [ctypes.c_void_p, ctypes.c_void_p, ctypes.c_uint64]
         _lib = lib
     return _lib
 
@@ -496,6 +500,25 @@ class Sdbg:
         self._check(self.lib.mgta_sdbg_unitig_copy(self.h, rp if U else None, U * 48, sp if C else None, C), "mgta_sdbg_unitig_copy")
         return rows, seq
 
+    # ---- the unitig graph (include/mgta_sdbg_unitig_graph.h) ----------------------------------------------------------
+    def unitig_links(self, device=False):
+        """the links between the rows of the last unitigs() call -> int64 [L, 2] (from, to), sorted: oriented unitigs
+        o = 2 * row (its sequence) or 2 * row + 1 (the reverse complement), one link of every twin pair, overlap k.
+        numpy, or a CUDA tensor on the graph's device when device=True."""
+        n = ctypes.c_int64()
+        self._check(self.lib.mgta_sdbg_unitig_links(self.h, ctypes.byref(n)), "mgta_sdbg_unitig_links")
+        L = n.value
+        if device:
+            import torch
+            links = torch.empty((L, 2), dtype=torch.int64, device="cuda:%d" % self.device)
+            torch.cuda.current_stream(links.device).synchronize()    # the copy runs on the graph's stream
+            p = links.data_ptr()
+        else:
+            links = np.empty((L, 2), np.int64)
+            p = links.ctypes.data
+        self._check(self.lib.mgta_sdbg_unitig_link_copy(self.h, p if L else None, L * 16), "mgta_sdbg_unitig_link_copy")
+        return links
+
 
 def pack_kmers(kmers, k):
     """ACGT strings of length k -> uint32 [n, ceil(2k / 32)]: the first character in bits 31..30 of word 0, unused low bits 0"""
@@ -542,6 +565,20 @@ def write_unitigs_fasta(path, rows, seq, min_len=0):
                 continue
             n, mult, flags = int(rows[i, 2]), int(rows[i, 4]), int(rows[i, 5])
             f.write(">unitig_%d len=%d edges=%d multi=%s flags=%d\n%s\n" % (i, len(s), n, "%.2f" % (mult / n) if mult >= 0 else "na", flags, s))
+
+
+def write_unitigs_gfa(path, rows, seq, links, k):
+    """the unitig graph as GFA 1.0 (Bandage and other GFA tools): one S line per row, named as in write_unitigs_fasta,
+    with KC:i:<mult_sum> when multiplicities are known, and one L line per link of Sdbg.unitig_links (+ for an even
+    oriented id, - for an odd one) with an overlap of k characters"""
+    rows, links = _host(rows), _host(links)
+    with open(path, "w") as f:
+        f.write("H\tVN:Z:1.0\n")
+        for i, s in enumerate(unitig_strings(rows, seq)):
+            mult = int(rows[i, 4])
+            f.write("S\tunitig_%d\t%s\tLN:i:%d%s\n" % (i, s, len(s), "\tKC:i:%d" % mult if mult >= 0 else ""))
+        for a, b in links.tolist():
+            f.write("L\tunitig_%d\t%s\tunitig_%d\t%s\t%dM\n" % (a // 2, "-" if a & 1 else "+", b // 2, "-" if b & 1 else "+", k))
 
 
 def pack_reads(seqs, device=0):

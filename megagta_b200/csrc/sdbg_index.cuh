@@ -63,11 +63,16 @@ struct mgta_sdbg {
     // first edge of every lv1 bucket (65536 + 1 entries, from the deliveries' bucket tables), and the queries' buffers
     std::vector<long long> bucket_start = std::vector<long long>(65537, 0);
     mgta_sdbg_impl::DevBuf q_bucket, q_in, q_out, q_err;
-    // unitigs (sdbg_unitig.cu): the rows and sequence of the last mgta_sdbg_unitigs, and its scratch (freed when it returns)
+    // unitigs (sdbg_unitig.cu): the rows and sequence of the last mgta_sdbg_unitigs, and its scratch (freed when it returns;
+    // mgta_sdbg_unitig_links takes its own scratch there too)
     mgta_sdbg_impl::DevBuf ut_rows, ut_seq, ut_edge, ut_seg, ut_jump;
     bool ut_ready = false;
     long long ut_n_rows = 0;
     unsigned long long ut_n_chars = 0;
+    // the links of the last mgta_sdbg_unitig_links, valid until the next mgta_sdbg_unitigs
+    mgta_sdbg_impl::DevBuf ul_links;
+    bool ul_ready = false;
+    long long ul_n_links = 0;
 };
 
 #define SCK(call)                                                                                        \

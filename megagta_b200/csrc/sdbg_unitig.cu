@@ -20,8 +20,17 @@
 //                 row order; k_ut_rows writes the rows, a scan of k + n the sequence offsets
 //   k_ut_scatter  every edge of a kept unitig writes its character; e1 also the k characters of LABEL(v(e1))
 // Scratch is int64 per edge and per ruler (edge ids pass 2^32) and is freed before mgta_sdbg_unitigs returns.
+//
+// The links between the unitigs (include/mgta_sdbg_unitig_graph.h), over the rows of the last mgta_sdbg_unitigs:
+//   k_ul_heads    one thread per row and side: id of every head (hid[first_edge] = 2r, hid[REVCOMP(last_edge)] = 2r + 1
+//                 for the partner of a row that is not its own reverse complement) and the partner's end REVCOMP(first_edge)
+//   k_ul_count    one thread per oriented unitig: FORWARD of its end, OUTGOING there, each out-edge through hid; counts
+//                 the canonical links.  scan of the counts = the output offsets in `from` order; k_ul_write repeats the
+//                 walk and writes the `to` values sorted inside the thread
+// Scratch is int64 per edge (hid) and per oriented unitig, and is freed before mgta_sdbg_unitig_links returns.
 #include "sdbg_nav.cuh"
 #include "../../include/mgta_sdbg_unitig.h"
+#include "../../include/mgta_sdbg_unitig_graph.h"
 
 using namespace mgta_sdbg_impl;
 
@@ -413,6 +422,96 @@ int unitigs(mgta_sdbg *g) {
     return MGTA_OK;
 }
 
+// ---- links between the unitigs ------------------------------------------------------------------------------------------
+__device__ __forceinline__ long long ul_bar(const long long *rows, long long o) { return (rows[(o >> 1) * 6 + 5] & 2) ? o : o ^ 1; }
+
+__global__ void __launch_bounds__(TPB, 4) k_ul_heads(const QueryParams P, long long U, const long long *rows, long long *hid,
+                                                  long long *end1) {
+    FOR_EACH(i, 2 * U) {
+        const long long r = i >> 1, *w = rows + r * 6;
+        const bool side = i & 1;
+        if (w[5] & 1) continue;                                    // a cycle has no head
+        if (!side) hid[w[0]] = 2 * r;
+        if (w[5] & 2) continue;
+        // one call site for both sides: a warp whose lanes took two calls would run them one after the other
+        const long long x = revcomp(P, w[side ? 0 : 1]);
+        if (side) end1[r] = x;
+        else if (x >= 0) hid[x] = 2 * r + 1;                       // x = -1 only for an invalid edge: never a row's last
+    }
+}
+
+// the canonical links out of oriented unitig o: their `to` values ascending in to[] -> their number (at most 4)
+__device__ __forceinline__ int ul_links_of(const QueryParams &P, const long long *rows, const long long *hid, const long long *end1,
+                                           long long o, long long *to) {
+    const long long r = o >> 1, fl = rows[r * 6 + 5];
+    if (fl & 1) {                                                  // a cycle: (2r, 2r) only
+        to[0] = o;
+        return (o & 1) ? 0 : 1;
+    }
+    if ((o & 1) && (fl & 2)) return 0;                             // a SELF_RC row has no 2r + 1
+    long long out[4];
+    const int n = outgoing(P, forward(P, (o & 1) ? end1[r] : rows[r * 6 + 1]), out);
+    const long long ba = ul_bar(rows, o);
+    int c = 0;
+    for (int j = 0; j < n; ++j) {
+        const long long b = hid[out[j]], bb = ul_bar(rows, b);
+        if (o < bb || (o == bb && b <= ba)) {                      // (o, b) <= (bar(b), bar(o))
+            int p = c++;
+            for (; p > 0 && to[p - 1] > b; --p) to[p] = to[p - 1];
+            to[p] = b;
+        }
+    }
+    return c;
+}
+
+__global__ void __launch_bounds__(TPB) k_ul_count(const QueryParams P, long long n_or, const long long *rows, const long long *hid,
+                                                  const long long *end1, long long *cnt) {
+    FOR_EACH(o, n_or) {
+        long long to[4];
+        cnt[o] = ul_links_of(P, rows, hid, end1, o, to);
+    }
+}
+
+__global__ void __launch_bounds__(TPB) k_ul_write(const QueryParams P, long long n_or, const long long *rows, const long long *hid,
+                                                  const long long *end1, const long long *off, long long *links) {
+    FOR_EACH(o, n_or) {
+        long long to[4];
+        const int n = ul_links_of(P, rows, hid, end1, o, to);
+        for (int j = 0; j < n; ++j) {
+            links[(off[o] + j) * 2] = o;
+            links[(off[o] + j) * 2 + 1] = to[j];
+        }
+    }
+}
+
+int unitig_links(mgta_sdbg *g) {
+    QueryParams P;
+    int rc;
+    if ((rc = query_params(g, &P))) return rc;
+    const long long E = g->n_edges, U = g->ut_n_rows, NO = 2 * U;
+    Scratch guard{g};
+    // hid per edge, end(2r + 1) per row, link counts per oriented unitig (NO + 1: the scan's total), the scan's tile sums
+    const size_t he = up256(8 * (size_t)E), hr = up256(8 * (size_t)U), ho = up256(8 * (size_t)(NO + 1));
+    const size_t nt = (size_t)(NO + SCAN_TILE - 1) / SCAN_TILE + 1;
+    if ((rc = grow(g, g->ut_edge, he + hr + ho + up256(8 * nt), 0))) return rc;
+    char *base = (char *)g->ut_edge.p;
+    long long *hid = (long long *)base, *end1 = (long long *)(base + he), *cnt = (long long *)(base + he + hr);
+    long long *tile_sum = (long long *)(base + he + hr + ho);
+    const long long *rows = (const long long *)g->ut_rows.p;
+    const unsigned go = grid_for(NO);
+    k_ul_heads<<<go, TPB, 0, g->stream>>>(P, U, rows, hid, end1);
+    k_ul_count<<<go, TPB, 0, g->stream>>>(P, NO, rows, hid, end1, cnt);
+    if ((rc = scan(g, cnt, NO, tile_sum))) return rc;
+    long long L = 0;
+    if ((rc = read_ll(g, cnt + NO, &L))) return rc;
+    if ((rc = grow(g, g->ul_links, 16 * (size_t)std::max(1ll, L), 0))) return rc;
+    k_ul_write<<<go, TPB, 0, g->stream>>>(P, NO, rows, hid, end1, cnt, (long long *)g->ul_links.p);
+    SCK(cudaGetLastError());
+    SCK(cudaStreamSynchronize(g->stream));
+    g->ul_n_links = L;
+    return MGTA_OK;
+}
+
 }  // namespace
 
 extern "C" int mgta_sdbg_unitigs(mgta_sdbg *g, int64_t *n_rows, uint64_t *n_chars) {
@@ -421,6 +520,7 @@ extern "C" int mgta_sdbg_unitigs(mgta_sdbg *g, int64_t *n_rows, uint64_t *n_char
     if (!g->finished) { g->err = "sdbg_unitigs: call mgta_sdbg_finish first"; return MGTA_ERR_STATE; }
     SCK(cudaSetDevice(g->device));
     g->ut_ready = false;
+    g->ul_ready = false;                                           // the links name rows of the previous call
     int rc;
     if ((rc = unitigs(g))) return rc;
     g->ut_ready = true;
@@ -449,6 +549,36 @@ extern "C" int mgta_sdbg_unitig_copy(mgta_sdbg *g, void *rows, uint64_t rows_byt
         SCK(cudaMemcpyAsync(rows, g->ut_rows.p, need_rows, on_device(rows) ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, g->stream));
     if (need_seq)
         SCK(cudaMemcpyAsync(seq, g->ut_seq.p, need_seq, on_device(seq) ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, g->stream));
+    SCK(cudaStreamSynchronize(g->stream));
+    return MGTA_OK;
+}
+
+extern "C" int mgta_sdbg_unitig_links(mgta_sdbg *g, int64_t *n_links) {
+    if (!g) return MGTA_ERR_ARG;
+    if (!n_links) { g->err = "sdbg_unitig_links: null n_links"; return MGTA_ERR_ARG; }
+    if (!g->ut_ready) { g->err = "sdbg_unitig_links: call mgta_sdbg_unitigs first"; return MGTA_ERR_STATE; }
+    SCK(cudaSetDevice(g->device));
+    g->ul_ready = false;
+    int rc;
+    if ((rc = unitig_links(g))) return rc;
+    g->ul_ready = true;
+    *n_links = g->ul_n_links;
+    return MGTA_OK;
+}
+
+extern "C" int mgta_sdbg_unitig_link_copy(mgta_sdbg *g, void *links, uint64_t bytes) {
+    if (!g) return MGTA_ERR_ARG;
+    if (!g->ul_ready) { g->err = "sdbg_unitig_link_copy: call mgta_sdbg_unitig_links after mgta_sdbg_unitigs first"; return MGTA_ERR_STATE; }
+    const uint64_t need = 16ull * (uint64_t)g->ul_n_links;
+    if (need && (!links || bytes < need)) {
+        char b[160];
+        snprintf(b, sizeof(b), "sdbg_unitig_link_copy: links buffer of %llu bytes, %llu needed", (unsigned long long)bytes, (unsigned long long)need);
+        g->err = b;
+        return MGTA_ERR_ARG;
+    }
+    SCK(cudaSetDevice(g->device));
+    if (need)
+        SCK(cudaMemcpyAsync(links, g->ul_links.p, need, on_device(links) ? cudaMemcpyDeviceToDevice : cudaMemcpyDeviceToHost, g->stream));
     SCK(cudaStreamSynchronize(g->stream));
     return MGTA_OK;
 }
